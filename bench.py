@@ -1,11 +1,14 @@
 #!/usr/bin/env python
-"""bench.py - headline benchmark of parakeet_b200 (contract in the task statement).
+"""bench.py - headline benchmark of parakeet_b200: one JSON result line on stdout.
 
 Workload (BASELINE.json configs[1]): Parallel WaveGAN generator inference, batch 32, 80-mel x 400 frames -> 3.84 M
 samples of 24 kHz audio per step, CSMSC generator (30 residual layers, 64/128 channels, upsample [4,5,3,5]), random
 weights of that architecture, synthetic N(0,1) mel + noise.  One step = one pass of the generator over one batch.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes the waveform the last timed step computed on rank 0 (B, 1, T float32, 15 MB) to DIR/wav.npy; the
+weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 N > 1 is launched by torchrun (one rank per GPU); utterances are independent, so every rank runs its own batch of 32
 with no data-path collective (weak scaling) and `value` is the whole-job aggregate.  The same line also carries, at every N,
@@ -313,6 +316,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the FastSpeech2 / end-to-end extras and the CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output (rank 0) to DIR/wav.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -379,6 +383,10 @@ def main():
     launches = lib.pk_launch_count() - launches0
     sampler.lines = sampler.lines[max(first_line - 1, 0):]      # samples taken during the timed region (+ the one straddling its start)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:        # before the sections below call gen again
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "wav.npy"), y.float().cpu().numpy())
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     layer_ms = [a.elapsed_time(b) for a, b in gen._layer_events]
     gen._layer_events = None

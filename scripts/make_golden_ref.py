@@ -3,12 +3,13 @@
 PaddlePaddle cannot be installed in the build container, so the reference cannot run as is.  Its model code is plain Python
 that calls ~60 Paddle primitives; `scripts/refexec/paddle_standin.py` maps those primitives onto torch (same mathematical
 definitions; the few Paddle-specific semantics are the ones oracle/README.md lists), `scripts/refexec/loader.py` imports the
-reference's files from /root/reference without running `parakeet/__init__.py`.  Under that stand-in this script builds the
+reference's files from a checkout of it without running `parakeet/__init__.py`.  Under that stand-in this script builds the
 reference's own FastSpeech2 / PWGGenerator / ConditionalWaveFlow classes, loads the oracle's seeded Paddle-layout state dicts
 into them (which also checks every state-dict key and shape against the reference's class tree) and records what the
-REFERENCE code computes.  tests/test_oracle_cpu.py then holds the oracle to these vectors.
+REFERENCE code computes.  tests/test_oracle_cpu.py then holds the oracle to these vectors.  Large arrays are stored as
+samples (tests/golden_sample.py) to keep the vectors small.
 
-    python scripts/make_golden_ref.py        # needs /root/reference; writes tests/golden/ref_executed*.npz
+    python scripts/make_golden_ref.py REFERENCE_DIR    # a PaddlePaddle/Parakeet checkout; writes tests/golden/ref_executed*.npz
 """
 import importlib.util
 import os
@@ -21,9 +22,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, HERE)
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+from golden_sample import compact  # noqa: E402
 from refexec import loader, paddle_standin  # noqa: E402
 
-REF = "/root/reference/parakeet"
+REF = None            # <REFERENCE_DIR>/parakeet, set by main()
 GOLD = os.path.join(ROOT, "tests", "golden")
 T = paddle_standin.T
 
@@ -91,6 +94,7 @@ def fastspeech2(out):
         out["fs2_inf_mel"] = ref.inference(T(xs[0])).numpy()
         out["fs2_inf_mel_alpha"] = ref.inference(T(xs[0]), alpha=1.3).numpy()        # uses the stand-in's round (restated)
         b = ofs.synth_train_batch(5, [23, 31, 17])
+        out["fs2_fwd_seed"] = np.asarray(5)
         for k, v in b.items():
             out[f"fs2_fwd_{k}"] = v.numpy()
         before, after, d_outs, p_outs, e_outs, ys, olens = ref(T(b["text"]), T(b["text_lengths"]), T(b["speech"]), T(b["speech_lengths"]),
@@ -127,6 +131,7 @@ def fastspeech2_multispeaker(out):
             # shape=[-1, T, -1], a -1 in a dimension that does not exist (fastspeech2.py:611-612) - speaker only there
             out[f"fs2ms_{tag}_inf_mel"] = ref.inference(T(xs[0]), spk_id=T(spk), tone_id=T(tone) if tt == "add" else None).numpy()
             b = ofs.synth_train_batch(22, [14, 19])
+            out[f"fs2ms_{tag}_fwd_seed"] = np.asarray(22)
             tone_b = torch.randint(0, 7, tuple(b["text"].shape), generator=g)
             spk_b = torch.tensor([1, 5])
             for k, v in b.items():
@@ -153,6 +158,7 @@ def fastspeech2_training(out):
     params = ofs.synth_params(1)
     ref.set_state_dict(params)
     b = ofs.synth_train_batch(9, [19, 27, 22])
+    out["fs2_train_seed"] = np.asarray(9)
     for k, v in b.items():
         out[f"fs2_train_{k}"] = v.numpy()
     before, after, d_outs, p_outs, e_outs, ys, olens = ref(T(b["text"]), T(b["text_lengths"]), T(b["speech"]), T(b["speech_lengths"]),
@@ -162,7 +168,7 @@ def fastspeech2_training(out):
                                                olens=olens)
     (l1 + dur + pitch + energy).backward()
     out["fs2_train_loss"] = np.asarray([float(l1), float(dur), float(pitch), float(energy)], dtype=np.float64)
-    # a representative subset of gradients (all 198 would be 150 MB): every kind of tensor on the path
+    # a representative subset of gradients (all 198 would be 150 MB): every kind of tensor on the path, + the L2 norm of each
     keep = ["encoder.embed.0.weight", "encoder.embed.1.alpha", "encoder.encoders.0.self_attn.linear_q.weight",
             "encoder.encoders.3.feed_forward.w_1.weight", "encoder.encoders.2.norm1.bias", "encoder.after_norm.weight",
             "duration_predictor.conv.0.0.weight", "duration_predictor.linear.bias", "pitch_predictor.conv.4.0.bias",
@@ -172,9 +178,8 @@ def fastspeech2_training(out):
     named = dict(ref.named_parameters())
     for k in keep:
         gk = named[k].grad
-        gk = (gk if gk is not None else torch.zeros_like(named[k])).detach().reshape(-1)
-        stride = max(1, gk.numel() // 20000)                          # big tensors: every stride-th element + the L2 norm
-        out["fs2_train_grad/" + k] = gk[::stride].numpy()
+        gk = (gk if gk is not None else torch.zeros_like(named[k])).detach()
+        out["fs2_train_grad/" + k] = gk.numpy()
         out["fs2_train_gradnorm/" + k] = np.asarray(float(gk.double().norm()))
     bufs = dict(ref.named_buffers())
     for k in ("postnet.postnet.0.1._mean", "postnet.postnet.0.1._variance", "postnet.postnet.4.1._variance"):
@@ -312,7 +317,11 @@ def wrappers_and_stft(out):
 
 
 def main():
-    uninstall = loader.install(paddle_standin.build())
+    global REF
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    REF = os.path.join(os.path.abspath(sys.argv[1]), "parakeet")
+    uninstall = loader.install(paddle_standin.build(), os.path.dirname(REF))
     try:
         small, models = {}, {}
         small_pieces(small)
@@ -325,6 +334,7 @@ def main():
         wrappers_and_stft(models)
     finally:
         uninstall()
+    models = compact(models, keep_full=("pwg_x", "stft_x", "mrstft_y", "wf2_z", "wf128_z"))   # inputs the tests read back
     np.savez(os.path.join(GOLD, "ref_executed.npz"), **small)
     np.savez_compressed(os.path.join(GOLD, "ref_executed_models.npz"), **models)
     for name, d in (("ref_executed.npz", small), ("ref_executed_models.npz", models)):

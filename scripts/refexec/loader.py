@@ -6,14 +6,15 @@ import os
 import sys
 import types
 
-REF_ROOT = "/root/reference"
-
 
 class _RefFinder(importlib.abc.MetaPathFinder):
+    def __init__(self, ref_root):
+        self.ref_root = ref_root
+
     def find_spec(self, name, path=None, target=None):
         if name != "parakeet" and not name.startswith("parakeet."):
             return None
-        rel = os.path.join(REF_ROOT, *name.split("."))
+        rel = os.path.join(self.ref_root, *name.split("."))
         if os.path.isdir(rel):
             spec = importlib.util.spec_from_loader(name, loader=None, is_package=True)
             spec.submodule_search_locations = [rel]
@@ -23,11 +24,11 @@ class _RefFinder(importlib.abc.MetaPathFinder):
         return None
 
 
-def install(standin_modules):
-    """Put the stand-in modules and the reference finder in place; returns an `uninstall()`."""
+def install(standin_modules, ref_root):
+    """Put the stand-in modules and a finder for the reference checkout at `ref_root` in place; returns an `uninstall()`."""
     saved = {k: sys.modules.get(k) for k in standin_modules}
     sys.modules.update(standin_modules)
-    finder = _RefFinder()
+    finder = _RefFinder(ref_root)
     sys.meta_path.insert(0, finder)
 
     def uninstall():
